@@ -11,6 +11,7 @@ the metric is quoted "@10M filters" and it fits one B200. Under torchrun every r
     python bench.py --gpus 1 --steps 20 --warmup 3
     python -m torch.distributed.run --nproc-per-node 8 ... bench.py --gpus 8
     python bench.py --impl reference        # the reference algorithm restated in C++ (oracle/), on host cores
+    python bench.py --dump-outputs DIR      # also write what the last timed step computed (seeded sample) as DIR/*.npy
 """
 import argparse
 import json
@@ -24,6 +25,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the source tree may be read-only: the bench writes nothing into it
 
 METRIC = "publish-topics matched/sec @10M filters"
 UNIT = "topics/s"
@@ -57,7 +59,13 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--max-pfanout", type=int, default=2 ** 31 - 1, help="Setting.MaxPersistentFanout (reference default INT_MAX)")
     ap.add_argument("--max-gfanout", type=int, default=100, help="Setting.MaxGroupFanout (reference default 100)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (a seeded sample of the batch) as DIR/<name>.npy, "
+                         "float64, under 64 MB in all: two builds run with the same arguments can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; --impl reference has none")
+    return args
 
 
 def dist_env():
@@ -212,13 +220,87 @@ def make_workload(args, rank, world):
     return Workload(args.config, scale=args.scale)
 
 
-def cpu_sample_indices(w, want):
-    """UNBIASED bounded sample of the batch: the whole batch when it fits `want`, else a uniform random subset without
+def cpu_sample_indices(n, want):
+    """UNBIASED bounded sample of a batch of n: the whole batch when it fits `want`, else a uniform random subset without
     replacement (seeded). Round 1 took "every topic of every 8th tenant", which over-weights the largest tenant (tenant index
     == Zipf rank): 1494 B/topic instead of the whole batch's 1162."""
-    if w.n_topics <= want:
-        return np.arange(w.n_topics)
-    return np.sort(np.random.default_rng(0xB1F20).choice(w.n_topics, want, replace=False))
+    if n <= want:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0xB1F20).choice(n, want, replace=False))
+
+
+# --dump-outputs: rows (topics, or filters for C5) of the seeded sample, values (route ranks / topic ids) kept of those rows, and
+# throttle events kept. Every array is float64 (its integers are exact there): at most 6 x 8 B x 65536 + 8 B x 3M + 24 B x 0.5M,
+# about 39 MB in all.
+DUMP_ROWS, DUMP_VALUES, DUMP_EVENTS = 1 << 16, 3_000_000, 500_000
+
+
+def sample_csr(offsets, values, pick, cap):
+    """rows `pick` (ascending) of a CSR whose values are unordered within a row (as bfq_expand_device leaves them) -> (offsets
+    over the picked rows, their values sorted within each row and cut after the first `cap`). torch tensors, any device;
+    values must lie in [0, 2^32)."""
+    import torch
+    lens = offsets[pick + 1] - offsets[pick]
+    out_off = torch.zeros(len(pick) + 1, dtype=torch.int64, device=offsets.device)
+    out_off[1:] = torch.cumsum(lens, 0)
+    total = int(out_off[-1])
+    row = torch.repeat_interleave(torch.arange(len(pick), device=offsets.device), lens)
+    pos = torch.arange(total, device=offsets.device) + (offsets[pick] - out_off[:-1])[row]
+    key = torch.sort((row << 32) | values[pos].to(torch.int64)).values[:cap]
+    return out_off, key & 0xFFFFFFFF
+
+
+def write_dump(out_dir, arrays):
+    """arrays (numpy or torch, any device) -> out_dir/<name>.npy in float64; an empty array is not written (no file says there
+    is nothing, e.g. no throttle event in the sample)"""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if not isinstance(a, np.ndarray):
+            a = a.cpu().numpy()
+        if a.size == 0:
+            continue
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
+def dump_forward(out_dir, res, dev, stream):
+    """the last timed step's bfq_match_device result, as its caller receives it, over a seeded sample of the batch's topics:
+    matched routes before caps and matched filters per topic, the surviving route ranks (caps applied: bfq_expand_device's
+    CSR, sorted within a topic), the number of throttle events per topic (persistent, group) and those events as
+    (topic, rank, kind) rows, sorted"""
+    import torch
+
+    from bifromq_b200 import dist as D
+    n = res.n_topics
+    d_off = torch.zeros(n + 1, dtype=torch.int64, device=dev)
+    total = res.expand(d_off.data_ptr(), None, 0, stream)
+    d_ranks = torch.zeros(max(total, 1), dtype=torch.int64, device=dev)
+    res.expand(d_off.data_ptr(), d_ranks.data_ptr(), total, stream)
+    torch.cuda.synchronize(dev)
+    pick = torch.from_numpy(cpu_sample_indices(n, DUMP_ROWS)).to(dev)
+    offsets, ranks = sample_csr(d_off, d_ranks, pick, DUMP_VALUES)
+    route_count = D.device_view(res.d_route_count, n, "<i4", dev)[pick]
+    span_count = D.device_view(res.d_span_count, n, "<i4", dev)[pick] & 0x3FFFFFFF   # the low 30 bits count the ranges
+    counts = torch.zeros((len(pick), 2), dtype=torch.int64, device=dev)
+    events = np.zeros((0, 3), np.int32)
+    if res.n_throttled:
+        ev = D.device_view(res.d_throttled, 3 * res.n_throttled, "<i4", dev).view(-1, 3)
+        slot = torch.full((n,), -1, dtype=torch.int64, device=dev)   # topic -> its position in the sample
+        slot[pick] = torch.arange(len(pick), device=dev)
+        ev = ev[slot[ev[:, 0].long()] >= 0]
+        counts = torch.bincount(2 * slot[ev[:, 0].long()] + (ev[:, 2] == 2), minlength=2 * len(pick)).view(-1, 2)   # kind 1 / 2
+        events = ev.cpu().numpy()
+        events = events[np.lexsort((events[:, 2], events[:, 1], events[:, 0]))][:DUMP_EVENTS]
+    write_dump(out_dir, {"topics": pick, "route_count": route_count, "span_count": span_count, "offsets": offsets, "ranks": ranks,
+                         "throttled_count": counts, "throttled": events})
+
+
+def dump_inverse(out_dir, res):
+    """the last timed step's bfq_rmatch result over a seeded sample of the query filters: total matches per filter and the
+    returned topic ids, sorted within a filter (under a limit, WHICH ids come back is left open, as in the reference)"""
+    import torch
+    pick = cpu_sample_indices(res.n_filters, DUMP_ROWS)
+    offsets, ids = sample_csr(torch.from_numpy(res.offsets), torch.from_numpy(res.ids), torch.from_numpy(pick), DUMP_VALUES)
+    write_dump(out_dir, {"filters": pick, "totals": res.totals[pick], "offsets": offsets, "ids": ids})
 
 
 _ORACLE_CACHE = {}
@@ -259,7 +341,7 @@ def run_cpu_baseline(w, args, mode_name, cached=False, n_passes=5, n_warm=0):
     matched once, the repeats are lookups."""
     cores = os.cpu_count() or 1
     want = args.cpu_sample or (1 << 30 if mode_name == "trie" else 100000)
-    idx = cpu_sample_indices(w, want)
+    idx = cpu_sample_indices(w.n_topics, want)
     O, kv, tenants, (pb, poff), tt = oracle_for_sample(w, idx)
     tb, toff = O.blob(tenants)
     n = len(idx)
@@ -452,6 +534,8 @@ def main_inverse(args, rank, world, local):
                             "counts_check": {"oracle_matches": matches, "gpu_matches": int(unl.totals.sum()), "equal": matches == int(unl.totals.sum())}}
         line["cpu_baseline"] = base
     print(json.dumps(line))
+    if args.dump_outputs:
+        dump_inverse(args.dump_outputs, last)
 
 
 def main():
@@ -734,6 +818,8 @@ def main():
         if cpu_base:
             line["cpu_baseline"] = cpu_base
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_forward(args.dump_outputs, out, dev, stream.cuda_stream)
     out.release()
     if world > 1:
         dist.barrier()

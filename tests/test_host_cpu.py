@@ -210,6 +210,33 @@ def test_bench_roofline_record_and_defaults():
     assert bench.pin_to_gpu_numa_node(0) is None      # no GPU here: must decline quietly, never raise
 
 
+def test_bench_dump_outputs_sample(tmp_path):
+    """bench.py --dump-outputs: the rows of the seeded sample are the same every run, each row's values come out sorted (the
+    device CSR leaves them unordered), the values are cut at the budget and the files are float64 .npy; an empty output (no
+    throttle event, say) is left out rather than written empty"""
+    import importlib.util
+    import torch
+    spec = importlib.util.spec_from_file_location("bench_module", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    rng = np.random.default_rng(1)
+    off = np.zeros(1001, np.int64)
+    off[1:] = np.cumsum(rng.integers(0, 9, 1000))
+    vals = rng.integers(0, 2 ** 32, int(off[-1]), dtype=np.int64)
+    pick = bench.cpu_sample_indices(1000, 100)
+    assert np.array_equal(pick, bench.cpu_sample_indices(1000, 100)) and len(np.unique(pick)) == 100
+    assert np.array_equal(bench.cpu_sample_indices(50, 100), np.arange(50))
+    got_off, got = bench.sample_csr(torch.from_numpy(off), torch.from_numpy(vals), torch.from_numpy(pick), 250)
+    rows = [sorted(vals[off[i]:off[i + 1]].tolist()) for i in pick]
+    assert got_off.tolist() == [0] + np.cumsum([len(r) for r in rows]).tolist()
+    flat = [v for r in rows for v in r]
+    assert len(flat) > 250 and got.tolist() == flat[:250]
+    bench.write_dump(str(tmp_path / "out"), {"offsets": got_off, "ranks": got, "topics": pick, "throttled": np.zeros((0, 3), np.int32)})
+    ranks = np.load(str(tmp_path / "out" / "ranks.npy"))
+    assert ranks.dtype == np.float64 and ranks.tolist() == flat[:250]
+    assert sorted(os.listdir(str(tmp_path / "out"))) == ["offsets.npy", "ranks.npy", "topics.npy"]
+
+
 def _route_blobs(pairs):
     keys = b"".join(k for k, _ in pairs)
     vals = b"".join(v for _, v in pairs)
